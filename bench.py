@@ -2,6 +2,7 @@
 """Benchmark of the UQ inference hot path (BASELINE.json metric: UQ samples x passes / sec).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload NAME]
+                    [--dump-outputs DIR]
 
 Workload (``configs[1]`` of BASELINE.json): binomial-options deep ensemble,
 16 members x (5 -> 512 -> 512 -> 512 -> 1, Linear+BatchNorm1d+ReLU), 1 M synthetic samples,
@@ -49,6 +50,7 @@ WORKLOADS = {
 }
 DEFAULT_WORKLOAD = "ensemble16x512_1M"
 N_ROTATE = 8  # input buffers rotated per step so the working set exceeds the 126 MB L2
+DUMP_BYTES = 64_000_000 - 4096  # --dump-outputs budget: 64 MB with room for the .npy headers
 
 
 def kernel_name(widths, d_out):
@@ -141,6 +143,7 @@ def cpu_forward_fn(workload, model):
 
 
 def time_cpu(workload, model, sample_n, steps, warmup):
+    """(rate, seconds per step, (mean, std) of the last timed step)"""
     mode, d_in, widths, d_out, k, n, p = WORKLOADS[workload]
     fn = cpu_forward_fn(workload, model)
     x = synth_x(sample_n, d_in, 0)
@@ -148,9 +151,9 @@ def time_cpu(workload, model, sample_n, steps, warmup):
         fn(x)
     t0 = time.perf_counter()
     for _ in range(steps):
-        fn(x)
+        out = fn(x)
     dt = (time.perf_counter() - t0) / steps
-    return sample_n * k / dt, dt
+    return sample_n * k / dt, dt, out
 
 
 def cpu_sample_size(workload):
@@ -178,11 +181,10 @@ def run_reference(args):
     mode, d_in, widths, d_out, k, n, p = WORKLOADS[wl]
     model = build_model(wl)
     sample_n = cpu_sample_size(wl)
-    steps, warmup = max(1, args.steps), max(1, min(args.warmup, 2))
-    # keep the whole run within a few minutes
-    probe_rate, probe_dt = time_cpu(wl, model, sample_n, 1, 1)
-    steps = max(1, min(steps, int(120.0 / max(probe_dt, 1e-3))))
-    rate, dt = time_cpu(wl, model, sample_n, steps, 0)
+    steps, warmup = args.steps, max(1, min(args.warmup, 2))
+    rate, dt, out = time_cpu(wl, model, sample_n, steps, warmup)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"mean": out[0], "std": out[1]})
     cores = torch.get_num_threads()
     line = {
         "impl": "reference", "metric": "uq_sample_passes_per_sec", "value": rate,
@@ -213,6 +215,18 @@ def config_dict(wl, n_gpus, sample_note=None):
     if sample_note:
         cfg["cpu_sample"] = sample_note
     return cfg
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: each array of the last timed step as ``out_dir/<name>.npy`` in float32, so
+    two builds run with the same arguments (hence the same seeded inputs) can be compared output
+    for output.  Above DUMP_BYTES in all, every array keeps the same evenly strided rows."""
+    import numpy as np
+    arrays = {name: a.detach().float().cpu().numpy() for name, a in arrays.items()}
+    stride = -(-sum(a.nbytes for a in arrays.values()) // DUMP_BYTES)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a[::stride]))
 
 
 # ------------------------------------------------------------------------------------------------
@@ -540,6 +554,8 @@ def run_gpu(args):
     wall = time.perf_counter() - t_wall0
     launches = ops.launch_count()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:   # every rank holds the whole (mean, std)
+        dump_outputs(args.dump_outputs, {"mean": out[0], "std": out[1]})
     total_ms = e_begin.elapsed_time(e_end)
     step_ms = [a.elapsed_time(b) for a, b in ev]
     t = torch.tensor([total_ms], dtype=torch.float64, device=dev)
@@ -701,7 +717,7 @@ def run_gpu(args):
         if world == 1 and not args.no_cpu_baseline:
             sample_n = cpu_sample_size(wl)
             cpu_model = build_model(wl)
-            rate, dt = time_cpu(wl, cpu_model, sample_n, 2, 1)
+            rate, dt, _ = time_cpu(wl, cpu_model, sample_n, 2, 1)
             line["cpu_baseline"] = {
                 "value": rate, "unit": "sample*members/s", "cores": torch.get_num_threads(),
                 "kind": "port",
@@ -732,7 +748,12 @@ def main():
                     help="skip timing the fp32 parity mode next to the bf16 line")
     ap.add_argument("--no-metric-kernels", action="store_true",
                     help="skip the Wasserstein / KDE-JS kernel timings added to the default line")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the (mean, std) of the last timed step as DIR/mean.npy and "
+                         "DIR/std.npy (float32, at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
     return run_gpu(args)

@@ -1,7 +1,7 @@
 """Import shims so the UNMODIFIED reference package can be imported in the authoring container.
 
-TEST INFRASTRUCTURE (oracle).  Used only by ``tests/golden/make_golden.py`` and by tests that
-are skipped when ``/root/reference`` is absent (it never exists on the GPU box).
+TEST INFRASTRUCTURE (oracle).  Used only by the ``tests/golden/make_golden*.py`` scripts that
+record the reference's outputs; the test-suite reads those recordings and never the reference.
 
 ``nnueehcs/models.py`` imports three modules that are not installed here and are not vendored
 in the reference tree (``models.py:2,3,8-9``): ``deltauq``, ``kde`` and ``pytorch_lightning``.

@@ -6,6 +6,7 @@ placement and train-mode flags :292-334).
 """
 import ctypes
 import io
+import json
 import os
 import pickle
 import re
@@ -264,59 +265,52 @@ def test_runtime_and_throughput_metrics_protocol():
     assert evaluation.EuclideanEvaluation()._evaluate_uncertainties(a, b) == {"euclidean_distance": 7.5}
 
 
-def test_host_side_metrics_have_the_reference_interface():
-    """Where /root/reference is present (the authoring container): the mirrored host-side metric
-    classes expose the reference's names, result keys, objectives, metric lists and factory
-    behaviour (evaluation.py:205-227, :383-516, :700-812)."""
-    from oracle import shims
-    if not shims.reference_available():
-        pytest.skip("reference tree not present")
-    _, _, ref = shims.import_reference()
+def test_host_side_metrics_have_the_reference_interface(golden_dir):
+    """The mirrored host-side metric classes expose the reference's names, result keys,
+    objectives, metric lists and factory behaviour (evaluation.py:205-227, :383-516, :700-812),
+    as recorded in tests/golden/host_metrics_interface.json (make_golden_interface.py)."""
+    with open(os.path.join(golden_dir, "host_metrics_interface.json")) as f:
+        ref = json.load(f)
 
     class Fake(torch.nn.Module):
         def forward(self, x, return_ue=False):
             return (x, x[:, 0]) if return_ue else x
 
     idd, ood = (torch.rand(20, 3), None), (torch.rand(20, 3), None)
-    for cls_name in ("BaseModelRuntimeEvaluation", "UncertaintyEstimatingRuntimeEvaluation",
-                     "BaseModelThroughputEvaluation", "UncertaintyEstimatingThroughputEvaluation"):
-        mine, theirs = getattr(evaluation, cls_name), getattr(ref, cls_name)
-        assert mine.name == theirs.name
-        assert mine.get_objectives() == theirs.get_objectives()
-        assert mine.get_metrics() == theirs.get_metrics()
-        a, b = mine(num_trials=2, num_warmup=1), theirs(num_trials=2, num_warmup=1)
-        assert a.get_name() == b.get_name()
-        if torch.cuda.is_available():      # the reference synchronises the device unconditionally
-            assert set(a.evaluate(Fake(), idd, ood)) == set(b.evaluate(Fake(), idd, ood))
-    assert evaluation.MaxMemoryUsageEvaluation.name == ref.MaxMemoryUsageEvaluation.name
+    assert sorted(ref["runtime_classes"]) == sorted(
+        ("BaseModelRuntimeEvaluation", "UncertaintyEstimatingRuntimeEvaluation",
+         "BaseModelThroughputEvaluation", "UncertaintyEstimatingThroughputEvaluation"))
+    for cls_name, theirs in ref["runtime_classes"].items():
+        mine = getattr(evaluation, cls_name)
+        assert mine.name == theirs["name"]
+        assert mine.get_objectives() == theirs["objectives"]
+        assert mine.get_metrics() == theirs["metrics"]
+        a = mine(num_trials=2, num_warmup=1)
+        assert a.get_name() == theirs["instance_name"]
+        assert sorted(a.evaluate(Fake(), idd, ood)) == theirs["result_keys"]
+    assert evaluation.MaxMemoryUsageEvaluation.name == ref["max_memory_usage"]["name"]
     assert (evaluation.MaxMemoryUsageEvaluation().get_objectives()
-            == ref.MaxMemoryUsageEvaluation().get_objectives())
-    ua = torch.rand(17, 4)
-    ub = torch.rand(17, 4)
-    got = evaluation.EuclideanEvaluation()._evaluate_uncertainties(
-        evaluation.UncertaintyEstimate(ua), evaluation.UncertaintyEstimate(ub))
-    exp = ref.EuclideanEvaluation()._evaluate_uncertainties(ref.UncertaintyEstimate(ua),
-                                                            ref.UncertaintyEstimate(ub))
-    assert got == exp
+            == ref["max_memory_usage"]["objectives"])
+
+    def scores(rows):
+        return evaluation.UncertaintyEstimate(torch.tensor(rows, dtype=torch.float32))
+
+    e = ref["euclidean"]
+    got = evaluation.EuclideanEvaluation()._evaluate_uncertainties(scores(e["a"]), scores(e["b"]))
+    assert got == e["result"]
     # JensenShannonEvaluation on [N, d > 1] scores: mean of scipy's jensenshannon over the rows
-    pa, pb = torch.rand(9, 4) + 0.1, torch.rand(9, 4) + 0.1
-    pa[0, 1] = 0.0
-    got = evaluation.JensenShannonEvaluation()._evaluate_uncertainties(
-        evaluation.UncertaintyEstimate(pa), evaluation.UncertaintyEstimate(pb))
-    exp = ref.JensenShannonEvaluation()._evaluate_uncertainties(ref.UncertaintyEstimate(pa),
-                                                                ref.UncertaintyEstimate(pb))
-    assert got["jensen_shannon_distance"] == pytest.approx(float(exp["jensen_shannon_distance"]),
-                                                           rel=1e-6)
-    cfg = [{"name": "uncertainty_estimating_throughput", "trials": 3, "warmup": 2},
-           {"name": "runtime", "trials": 4}, {"name": "max_memory_usage"}, {"name": "mean_score"}]
-    mine, theirs = evaluation.get_evaluator(cfg), ref.get_evaluator(cfg)
-    assert [type(m).__name__ for m in mine.metrics] == [type(m).__name__ for m in theirs.metrics]
-    assert [(getattr(m, "num_trials", None), getattr(m, "num_warmup", None)) for m in mine.metrics] \
-        == [(getattr(m, "num_trials", None), getattr(m, "num_warmup", None)) for m in theirs.metrics]
-    ucfg = [{"name": "runtime", "trials": 4}, "uncertainty_estimating_runtime", "euclidean_distance",
-            {"name": "uncertainty_estimating_throughput", "warmup": 1}]
-    mine, theirs = evaluation.get_uncertainty_evaluator(ucfg), ref.get_uncertainty_evaluator(ucfg)
-    assert [type(m).__name__ for m in mine.metrics] == [type(m).__name__ for m in theirs.metrics]
+    j = ref["jensen_shannon"]
+    got = evaluation.JensenShannonEvaluation()._evaluate_uncertainties(scores(j["a"]), scores(j["b"]))
+    assert got["jensen_shannon_distance"] == pytest.approx(
+        j["result"]["jensen_shannon_distance"], rel=1e-6)
+    g = ref["get_evaluator"]
+    mine = evaluation.get_evaluator(g["config"])
+    assert [type(m).__name__ for m in mine.metrics] == g["classes"]
+    assert [[getattr(m, "num_trials", None), getattr(m, "num_warmup", None)] for m in mine.metrics] \
+        == g["trials_warmup"]
+    g = ref["get_uncertainty_evaluator"]
+    mine = evaluation.get_uncertainty_evaluator(g["config"])
+    assert [type(m).__name__ for m in mine.metrics] == g["classes"]
 
 
 def test_split_blocks_vocabulary(descr):
