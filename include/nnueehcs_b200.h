@@ -133,7 +133,8 @@ int uq_model_destroy(uq_model_t* model);
 /* 1 if the bf16 tcgen05 path supports this model's shapes, else 0 (reason in uq_last_error) */
 int uq_model_supports_bf16(const uq_model_t* model);
 /* 1 if UQ_PREC_FP32 runs on the tensor cores for this model (equal hidden widths, multiple of 64,
-   <= 512, at most 21 network inputs), else 0 (reason in uq_last_error) and UQ_PREC_FP32 is the
+   <= 512, at most 16 network inputs -- for UQ_MODE_DELTA_UQ / UQ_MODE_PAGER that is the doubled
+   width, so at most 8 sample features), else 0 (reason in uq_last_error) and UQ_PREC_FP32 is the
    CUDA-core path */
 int uq_model_supports_fp32_tc(const uq_model_t* model);
 

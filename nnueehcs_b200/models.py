@@ -17,6 +17,11 @@ Knobs that do not exist in the reference (all optional, attributes on the wrappe
                   CUDA-core FFMA for shapes the split kernels do not cover) or ``'bf16'`` (tcgen05
                   tensor-core mode); default overridable with ``NNUEEHCS_B200_PRECISION``.
 ``uq_shard``      optional ``distributed.KShard`` -- shard members/passes/anchors over ranks.
+
+float64 callers (a model cast with ``.double()`` and float64 inputs, as ``bo.py`` does with the
+dataset's dtype) get float64 outputs, but the forward computes in fp32: with ``'fp32'`` the results
+are within the fp32 bound, ``1e-5 * |ref| + 1e-5 * max|ref_mean|``, of a float64 reference -- not
+float64 accuracy.
 """
 from __future__ import annotations
 

@@ -11,7 +11,7 @@ fp32 mode : north_star's 1e-5 relative, read as ``|got-ref| <= 1e-5*|ref| + 1e-5
             ``precision='fp32'`` is the tensor-core split kernel (csrc/mlp_tcx.cu) wherever the model
             is eligible and the CUDA-core path otherwise; ``'fp32_ffma'`` forces the CUDA-core path.
             Both are held to the same 1e-5.
-bf16 mode : stated tolerance (``_bf16_check``): mean and std within ``1e-2 * scale`` with
+bf16 mode : stated tolerance (``tests.util.bf16_check``): mean and std within ``1e-2 * scale`` with
             ``scale = max|ref_mean| + max|ref_std|`` (the size of one member's output; measured worst
             case 2.3e-3 .. 4.3e-3), and the std within ``5e-2`` of its own scale (measured <= 2.2e-2).
             bf16 rounds weights and activations to 8 bits once per layer.  Measured errors are printed.
@@ -26,8 +26,9 @@ from nnueehcs_b200 import ops
 from nnueehcs_b200.model_builder import (DeltaUQMLPModelBuilder, EnsembleModelBuilder,
                                          MCDropoutModelBuilder, build_network)
 from oracle import uq_oracle
-from tests.util import (assert_close_ref, delta_arch, golden_arch, golden_masks, injected_to_masks,
-                        load_golden, masks_to_injected, mc_arch_with_dropout, nets_from_golden)
+from tests.util import (assert_close_ref, bf16_check, delta_arch, golden_arch, golden_masks,
+                        injected_to_masks, load_golden, masks_to_injected, mc_arch_with_dropout,
+                        nets_from_golden, randomise_bn, wide_arch)
 
 pytestmark = pytest.mark.gpu
 DEV = torch.device("cuda:0")
@@ -35,29 +36,6 @@ RTOL32 = 1e-5
 
 
 FP32_MODES = ["fp32", "fp32_ffma"]
-
-
-def _bf16_check(mean, std, ref_mean, ref_std, what, tol=1e-2, tol_std=5e-2):
-    """bf16 tolerance.  The natural unit is the magnitude of one member's output, taken as
-    ``scale = max|ref_mean| + max|ref_std|``: both errors must stay within ``tol * scale`` (measured
-    worst case over every bf16 test: 2.3e-3, and 4.3e-3 for identical passes whose std is 0 -- the
-    bound is 2.5-5x that; a mis-addressed K chunk is an error of >= 1/8 of scale), and the std
-    additionally within ``tol_std`` of its OWN scale (measured 1e-3 .. 2.2e-2; the largest values
-    belong to anchored nets whose spread is 16x smaller than their mean)."""
-    mean, std = mean.double().cpu(), std.double().cpu()
-    ref_mean, ref_std = torch.as_tensor(ref_mean).double(), torch.as_tensor(ref_std).double()
-    ms, ss = float(ref_mean.abs().max()), float(ref_std.abs().max())
-    scale = ms + ss
-    e_mean = float((mean - ref_mean).abs().max())
-    e_std = float((std - ref_std).abs().max())
-    print(f"[bf16 {what}] max|mean err| = {e_mean:.3e} ({e_mean / scale:.3e} of scale), "
-          f"max|std err| = {e_std:.3e} ({e_std / scale:.3e} of scale, "
-          f"{e_std / max(ss, 1e-30):.3e} of std scale)")
-    assert e_mean <= tol * scale, f"{what}: bf16 mean error {e_mean / scale:.3e} of scale > {tol}"
-    assert e_std <= tol * scale, f"{what}: bf16 std error {e_std / scale:.3e} of scale > {tol}"
-    if ss > 1e-3 * ms:   # identical passes have std == 0: nothing relative to check
-        assert e_std <= tol_std * ss, \
-            f"{what}: bf16 std error {e_std / ss:.3e} of std scale > {tol_std}"
 
 
 # ---- ensemble -----------------------------------------------------------------------------------
@@ -83,7 +61,7 @@ def test_ensemble_bf16_within_stated_tolerance(name):
     assert packed.supports_bf16, packed.bf16_reason
     x = torch.from_numpy(g["x"]).to(DEV)
     mean, std = packed.forward(x, "ensemble", total_members=k, precision="bf16")
-    _bf16_check(mean, std, g["mean"], g["std"], name)
+    bf16_check(mean, std, g["mean"], g["std"], name)
 
 
 def test_bf16_rejects_unsupported_shapes_loudly():
@@ -167,10 +145,10 @@ def test_mc_dropout_bf16_injected_masks():
     inj = masks_to_injected(golden_masks(g)).to(DEV)
     mean, std = packed.forward(x, "mc_dropout", total_members=passes, precision="bf16",
                                dropout_p=p, masks=inj)
-    _bf16_check(mean, std, g["mean"], g["std"], "mcdropout_binomial injected")
+    bf16_check(mean, std, g["mean"], g["std"], "mcdropout_binomial injected")
     mean0, std0 = packed.forward(x, "mc_dropout", total_members=passes, precision="bf16",
                                  dropout_p=p, dropout_active=False)
-    _bf16_check(mean0, std0, g["mean_off"], g["std_off"], "mcdropout_binomial off")
+    bf16_check(mean0, std0, g["mean_off"], g["std_off"], "mcdropout_binomial off")
 
 
 @pytest.mark.parametrize("precision", ["fp32", "fp32_ffma", "bf16"])
@@ -193,7 +171,7 @@ def test_mc_dropout_native_philox_replays_exactly_through_oracle(precision):
         assert_close_ref(mean, ref_mean, RTOL32, what="philox replay mean")
         assert_close_ref(std, ref_std, RTOL32, scale_ref=ref_mean, what="philox replay std")
     else:
-        _bf16_check(mean, std, ref_mean, ref_std, "philox replay")
+        bf16_check(mean, std, ref_mean, ref_std, "philox replay")
     # and feeding the exported masks back as injected masks gives the identical result
     mean_i, std_i = packed.forward(x, "mc_dropout", total_members=passes, precision=precision,
                                    dropout_p=p, masks=flat)
@@ -266,7 +244,7 @@ def test_delta_uq_matches_restatement(precision):
         assert_close_ref(mean, ref_mean, RTOL32, what="delta mean")
         assert_close_ref(std, ref_std, RTOL32, scale_ref=ref_mean, what="delta std")
     else:
-        _bf16_check(mean, std, ref_mean, ref_std, "delta_uq")
+        bf16_check(mean, std, ref_mean, ref_std, "delta_uq")
 
 
 def test_delta_uq_wrapper():
@@ -367,7 +345,7 @@ def test_pager_narrow_and_wide_kernels_bf16():
     kernel), 2x768 (wide kernel); ragged N, K = 7 anchors."""
     for width, depth, n in ((128, 6, 1000), (256, 3, 700), (768, 2, 300)):
         torch.manual_seed(width)
-        net = build_network(delta_arch(_wide_arch(5, width, depth, 1))).eval()
+        net = build_network(delta_arch(wide_arch(5, width, depth, 1))).eval()
         x, anchors, ys = torch.rand(n, 5), torch.rand(7, 5), torch.rand(7, 1) * 0.2
         packed = ops.PackedModel([net], DEV)
         assert packed.supports_bf16
@@ -417,7 +395,7 @@ def test_ragged_sample_counts(precision, n):
         assert_close_ref(mean, ref_mean, RTOL32, what=f"n={n} mean")
         assert_close_ref(std, ref_std, RTOL32, scale_ref=ref_mean, what=f"n={n} std")
     else:
-        _bf16_check(mean, std, ref_mean, ref_std, f"n={n}")
+        bf16_check(mean, std, ref_mean, ref_std, f"n={n}")
 
 
 def test_many_passes_few_samples_uses_member_splits():
@@ -432,7 +410,7 @@ def test_many_passes_few_samples_uses_member_splits():
                               dropout_p=p, seed=seed)
     m16, s16 = packed.forward(x, "mc_dropout", total_members=passes, precision="bf16",
                               dropout_p=p, seed=seed)
-    _bf16_check(m16, s16, m32.cpu(), s32.cpu(), "member splits")
+    bf16_check(m16, s16, m32.cpu(), s32.cpu(), "member splits")
 
 
 def test_single_member_std_is_nan_like_torch():
@@ -481,41 +459,21 @@ def test_host_buffer_entry_point():
 
 # ---- wide nets (hidden width 768 / 1024): the 64-rows-per-CTA pair kernel, mlp_tc3.cu -----------
 
-def _wide_arch(d_in, width, n_hidden, d_out, bn=True):
-    arch, prev = [], d_in
-    for _ in range(n_hidden):
-        arch.append({"Linear": {"args": [prev, width]}})
-        if bn:
-            arch.append({"BatchNorm1d": {"args": [width]}})
-        arch.append({"ReLU": {"inplace": True}})
-        prev = width
-    arch.append({"Linear": {"args": [prev, d_out]}})
-    return arch
-
-
-def _randomise_bn(net, seed):
-    gen = torch.Generator().manual_seed(seed)
-    for m in net.modules():
-        if isinstance(m, torch.nn.BatchNorm1d):
-            m.running_mean.copy_(torch.randn(m.num_features, generator=gen) * 0.1)
-            m.running_var.copy_(torch.rand(m.num_features, generator=gen) + 0.5)
-
-
 @pytest.mark.parametrize("width,n_hidden,k,n,d_out", [(1024, 2, 3, 300, 1), (1024, 7, 2, 129, 1),
                                                       (768, 3, 2, 64, 3)])
 def test_wide_ensemble_bf16(width, n_hidden, k, n, d_out):
     nets = []
     for i in range(k):
         torch.manual_seed(42 + i)
-        net = build_network(_wide_arch(5, width, n_hidden, d_out)).eval()
-        _randomise_bn(net, 1 + i)
+        net = build_network(wide_arch(5, width, n_hidden, d_out)).eval()
+        randomise_bn(net, 1 + i)
         nets.append(net)
     x = torch.rand(n, 5, generator=torch.Generator().manual_seed(0))
     packed = ops.PackedModel(nets, DEV)
     assert packed.supports_bf16, packed.bf16_reason
     mean, std = packed.forward(x.to(DEV), "ensemble", total_members=k, precision="bf16")
     ref_mean, ref_std = uq_oracle.ensemble_forward(nets, x)
-    _bf16_check(mean, std, ref_mean, ref_std, f"wide ensemble {width}x{n_hidden}")
+    bf16_check(mean, std, ref_mean, ref_std, f"wide ensemble {width}x{n_hidden}")
     # K-axis shards of the same forward merge to the same result
     m_a, s_a = packed.forward(x.to(DEV), "ensemble", total_members=k, precision="bf16",
                               member_begin=0, member_count=1, output="moments")
@@ -529,8 +487,8 @@ def test_wide_ensemble_bf16(width, n_hidden, k, n, d_out):
 def test_wide_mc_dropout_philox_replays_through_oracle():
     p, passes, seed, n = 0.2, 6, 77, 150
     torch.manual_seed(42)
-    net = build_network(mc_arch_with_dropout(_wide_arch(5, 1024, 3, 1), p)).eval()
-    _randomise_bn(net, 1)
+    net = build_network(mc_arch_with_dropout(wide_arch(5, 1024, 3, 1), p)).eval()
+    randomise_bn(net, 1)
     packed = ops.PackedModel([net], DEV)
     assert packed.supports_bf16, packed.bf16_reason
     x_cpu = torch.rand(n, 5, generator=torch.Generator().manual_seed(5))
@@ -539,7 +497,7 @@ def test_wide_mc_dropout_philox_replays_through_oracle():
     flat = ops.philox_keep_masks(n, packed.dropout_widths, passes, p, seed, 0, DEV)
     masks = injected_to_masks(flat.cpu(), n, packed.dropout_widths, passes)
     ref_mean, ref_std = uq_oracle.mc_dropout_forward(net, x_cpu, passes, p, masks=masks)
-    _bf16_check(mean, std, ref_mean, ref_std, "wide philox replay")
+    bf16_check(mean, std, ref_mean, ref_std, "wide philox replay")
     mean_i, std_i = packed.forward(x_cpu.to(DEV), "mc_dropout", total_members=passes,
                                    precision="bf16", dropout_p=p, masks=flat)
     assert torch.equal(mean, mean_i) and torch.equal(std, std_i)
@@ -553,15 +511,15 @@ def test_wide_mc_dropout_philox_replays_through_oracle():
 def test_wide_delta_uq_bf16():
     k, n = 4, 200
     torch.manual_seed(42)
-    net = build_network(delta_arch(_wide_arch(5, 768, 2, 1))).eval()
-    _randomise_bn(net, 1)
+    net = build_network(delta_arch(wide_arch(5, 768, 2, 1))).eval()
+    randomise_bn(net, 1)
     packed = ops.PackedModel([net], DEV)
     x = torch.rand(n, 5, generator=torch.Generator().manual_seed(2))
     anchors = torch.rand(k, 5, generator=torch.Generator().manual_seed(3))
     mean, std = packed.forward(x.to(DEV), "delta_uq", total_members=k, precision="bf16",
                                anchors=anchors.to(DEV))
     ref_mean, ref_std = uq_oracle.delta_uq_forward(net, x, anchors, k)
-    _bf16_check(mean, std, ref_mean, ref_std, "wide delta_uq")
+    bf16_check(mean, std, ref_mean, ref_std, "wide delta_uq")
 
 
 # ---- every kernel family at awkward sizes --------------------------------------------------------
@@ -582,15 +540,15 @@ def test_bf16_kernels_at_ragged_sizes(width, n_hidden, n, k):
     nets = []
     for i in range(k):
         torch.manual_seed(100 + i)
-        net = build_network(_wide_arch(7, width, n_hidden, 1)).eval()
-        _randomise_bn(net, 50 + i)
+        net = build_network(wide_arch(7, width, n_hidden, 1)).eval()
+        randomise_bn(net, 50 + i)
         nets.append(net)
     x = torch.rand(n, 7, generator=torch.Generator().manual_seed(n))
     packed = ops.PackedModel(nets, DEV)
     assert packed.supports_bf16, packed.bf16_reason
     mean, std = packed.forward(x.to(DEV), "ensemble", total_members=k, precision="bf16")
     ref_mean, ref_std = uq_oracle.ensemble_forward(nets, x)
-    _bf16_check(mean, std, ref_mean, ref_std, f"ragged {width}x{n_hidden} n={n}")
+    bf16_check(mean, std, ref_mean, ref_std, f"ragged {width}x{n_hidden} n={n}")
     # the same rows inside a larger batch give bit-identical results (tiles are independent)
     xb = torch.cat([x, torch.rand(300, 7, generator=torch.Generator().manual_seed(1))])
     mean_b, std_b = packed.forward(xb.to(DEV), "ensemble", total_members=k, precision="bf16")
@@ -677,7 +635,7 @@ def test_pager_multi_output_and_anchor_prefix(precision):
     kernel), more anchor rows stored than num_anchors uses, and a K-range call that covers only the
     last anchors (member_begin > 0: targets / per-anchor biases are indexed by the GLOBAL id)."""
     torch.manual_seed(3)
-    net = build_network(delta_arch(_wide_arch(4, 128, 3, 3))).eval()
+    net = build_network(delta_arch(wide_arch(4, 128, 3, 3))).eval()
     x, anchors, ys = torch.rand(500, 4), torch.rand(9, 4), torch.rand(9, 3) * 0.3
     k = 6
     packed = ops.PackedModel([net], DEV)
@@ -713,10 +671,10 @@ def test_fp32_runs_on_the_tensor_cores_where_eligible():
     packed = ops.PackedModel(nets_from_golden(g, int(g["k"])), DEV)
     assert not packed.fp32_on_tensor_cores and "hidden" in packed.fp32_tc_reason
     torch.manual_seed(0)                       # 1024-wide: no room for two fp16 pieces of a tile
-    packed = ops.PackedModel([build_network(_wide_arch(5, 1024, 2, 1)).eval()], DEV)
+    packed = ops.PackedModel([build_network(wide_arch(5, 1024, 2, 1)).eval()], DEV)
     assert not packed.fp32_on_tensor_cores and "512" in packed.fp32_tc_reason
     torch.manual_seed(0)                       # 17 inputs: the layer-0 chunk holds at most 16
-    packed = ops.PackedModel([build_network(_wide_arch(17, 128, 2, 1)).eval()], DEV)
+    packed = ops.PackedModel([build_network(wide_arch(17, 128, 2, 1)).eval()], DEV)
     assert not packed.fp32_on_tensor_cores and "16" in packed.fp32_tc_reason
 
 
@@ -724,13 +682,14 @@ def test_fp32_runs_on_the_tensor_cores_where_eligible():
     (64, 2, 1, 2, 5, 1), (64, 3, 1025, 3, 7, 1), (128, 1, 300, 2, 5, 1), (128, 6, 2049, 2, 5, 1),
     (192, 2, 257, 2, 16, 1), (256, 3, 130, 4, 5, 3), (320, 2, 383, 2, 9, 1), (384, 2, 200, 2, 5, 8),
     (448, 2, 129, 2, 5, 1), (512, 3, 4097, 4, 5, 1), (512, 2, 65, 2, 12, 2),
+    (128, 2, 259, 3, 16, 1),   # four-slot split kernel, layer 0 built in place (K0 = 64)
 ])
 def test_fp32_split_kernel_all_widths(width, n_hidden, n, k, d_in, d_out):
     nets = []
     for i in range(k):
         torch.manual_seed(100 + i)
-        net = build_network(_wide_arch(d_in, width, n_hidden, d_out)).eval()
-        _randomise_bn(net, 50 + i)
+        net = build_network(wide_arch(d_in, width, n_hidden, d_out)).eval()
+        randomise_bn(net, 50 + i)
         nets.append(net)
     # unnormalised inputs on purpose: the row scales must absorb them
     x = torch.rand(n, d_in, generator=torch.Generator().manual_seed(n)) * 37.0 - 11.0
@@ -751,7 +710,7 @@ def test_fp32_split_kernel_is_scale_free(scale):
     """Activations far from 1 (tiny / huge weights and inputs): the power-of-two row and weight
     scales keep every fp16 piece in range, so the result tracks the reference at any magnitude."""
     torch.manual_seed(7)
-    net = build_network(_wide_arch(5, 256, 3, 1, bn=False)).eval()
+    net = build_network(wide_arch(5, 256, 3, 1, bn=False)).eval()
     with torch.no_grad():
         net[0].weight.mul_(scale)
         net[0].bias.mul_(scale)
@@ -770,11 +729,11 @@ def test_dropout_before_the_final_linear():
     reference's builder never makes one, model_builder.py:257-262): its 1 / (1 - p) applies to the
     final dot product in every kernel."""
     p, passes, seed, n = 0.25, 10, 11, 200
-    arch = mc_arch_with_dropout(_wide_arch(5, 128, 3, 1), p)
+    arch = mc_arch_with_dropout(wide_arch(5, 128, 3, 1), p)
     arch.insert(len(arch) - 1, {"Dropout": {"args": [p]}})
     torch.manual_seed(42)
     net = build_network(arch).eval()
-    _randomise_bn(net, 1)
+    randomise_bn(net, 1)
     packed = ops.PackedModel([net], DEV)
     x_cpu = torch.rand(n, 5, generator=torch.Generator().manual_seed(5))
     flat = ops.philox_keep_masks(n, packed.dropout_widths, passes, p, seed, 0, DEV)
@@ -784,7 +743,7 @@ def test_dropout_before_the_final_linear():
         mean, std = packed.forward(x_cpu.to(DEV), "mc_dropout", total_members=passes,
                                    precision=precision, dropout_p=p, seed=seed)
         if precision == "bf16":
-            _bf16_check(mean, std, ref_mean, ref_std, "dropout before final Linear")
+            bf16_check(mean, std, ref_mean, ref_std, "dropout before final Linear")
         else:
             assert_close_ref(mean, ref_mean, RTOL32, what=f"{precision} mean")
             assert_close_ref(std, ref_std, RTOL32, scale_ref=ref_mean, what=f"{precision} std")
@@ -796,8 +755,8 @@ def _baseline_nets(d_in, width, n_hidden, k, d_out=1):
     nets = []
     for i in range(k):
         torch.manual_seed(42 + i)            # model_builder.py:229 seeds member i with 42 + i
-        net = build_network(_wide_arch(d_in, width, n_hidden, d_out)).eval()
-        _randomise_bn(net, 1 + i)
+        net = build_network(wide_arch(d_in, width, n_hidden, d_out)).eval()
+        randomise_bn(net, 1 + i)
         nets.append(net)
     return nets
 
@@ -816,8 +775,8 @@ def test_baseline_config1_ensemble16x512():
     assert_close_ref(mean, ref_mean, RTOL32, what="cfg1 fp32 mean")
     assert_close_ref(std, ref_std, RTOL32, scale_ref=ref_mean, what="cfg1 fp32 std")
     mean, std = packed.forward(x.to(DEV), "ensemble", total_members=k, precision="bf16")
-    _bf16_check(mean, std, ref_mean, ref_std, "cfg1 bf16")
-    model = EnsembleModelBuilder(_wide_arch(5, 512, 3, 1), {"num_models": k}).build()
+    bf16_check(mean, std, ref_mean, ref_std, "cfg1 bf16")
+    model = EnsembleModelBuilder(wide_arch(5, 512, 3, 1), {"num_models": k}).build()
     for m, ref in zip(model.models, nets):
         m.load_state_dict(ref.state_dict())
     model.to(DEV).eval()
@@ -836,8 +795,8 @@ def test_baseline_config2_deltauq_32_anchors_6x128():
     (oracle restatement), like every Delta-UQ check."""
     k, n = 32, 20011
     torch.manual_seed(42)
-    net = build_network(delta_arch(_wide_arch(5, 128, 6, 1))).eval()
-    _randomise_bn(net, 1)
+    net = build_network(delta_arch(wide_arch(5, 128, 6, 1))).eval()
+    randomise_bn(net, 1)
     x = torch.rand(n, 5, generator=torch.Generator().manual_seed(0))
     anchors = torch.rand(k, 5, generator=torch.Generator().manual_seed(2))
     ref_mean, ref_std = uq_oracle.delta_uq_forward(net, x, anchors, k)
@@ -849,8 +808,8 @@ def test_baseline_config2_deltauq_32_anchors_6x128():
     assert_close_ref(std, ref_std, RTOL32, scale_ref=ref_mean, what="cfg2 fp32 std")
     mean, std = packed.forward(x.to(DEV), "delta_uq", total_members=k, precision="bf16",
                                anchors=anchors.to(DEV))
-    _bf16_check(mean, std, ref_mean, ref_std, "cfg2 bf16")
-    model = DeltaUQMLPModelBuilder(_wide_arch(5, 128, 6, 1), {"estimator": "std", "num_anchors": k,
+    bf16_check(mean, std, ref_mean, ref_std, "cfg2 bf16")
+    model = DeltaUQMLPModelBuilder(wide_arch(5, 128, 6, 1), {"estimator": "std", "num_anchors": k,
                                                               "anchored_batch_size": 4096}).build()
     model.net.load_state_dict(net.state_dict())
     model.anchors = anchors
@@ -867,8 +826,8 @@ def test_baseline_config3_mcdropout_8x1024_philox_replay():
     CUDA-core path (fp32; width 1024 has no split kernel)."""
     p, passes, seed, n = 0.2, 8, 20261018, 1500
     torch.manual_seed(42)
-    net = build_network(mc_arch_with_dropout(_wide_arch(5, 1024, 7, 1), p)).eval()
-    _randomise_bn(net, 1)
+    net = build_network(mc_arch_with_dropout(wide_arch(5, 1024, 7, 1), p)).eval()
+    randomise_bn(net, 1)
     packed = ops.PackedModel([net], DEV)
     x_cpu = torch.rand(n, 5, generator=torch.Generator().manual_seed(5))
     flat = ops.philox_keep_masks(n, packed.dropout_widths, passes, p, seed, 0, DEV)
@@ -880,8 +839,8 @@ def test_baseline_config3_mcdropout_8x1024_philox_replay():
     assert_close_ref(std, ref_std, RTOL32, scale_ref=ref_mean, what="cfg3 fp32 std")
     mean, std = packed.forward(x_cpu.to(DEV), "mc_dropout", total_members=passes, precision="bf16",
                                dropout_p=p, seed=seed)
-    _bf16_check(mean, std, ref_mean, ref_std, "cfg3 bf16")
-    model = MCDropoutModelBuilder(_wide_arch(5, 1024, 7, 1), {"num_samples": passes,
+    bf16_check(mean, std, ref_mean, ref_std, "cfg3 bf16")
+    model = MCDropoutModelBuilder(wide_arch(5, 1024, 7, 1), {"num_samples": passes,
                                                               "dropout_percent": p}).build()
     model.model.load_state_dict(net.state_dict())
     model.to(DEV).eval()
@@ -923,7 +882,7 @@ def test_wide_ensemble_split_major_member_groups():
     packed = ops.PackedModel(nets, DEV)
     mean, std = packed.forward(x.to(DEV), "ensemble", total_members=k, precision="bf16")
     ref_mean, ref_std = uq_oracle.ensemble_forward(nets, x)
-    _bf16_check(mean, std, ref_mean, ref_std, "split-major wide ensemble")
+    bf16_check(mean, std, ref_mean, ref_std, "split-major wide ensemble")
     # the same forward as two K-shards (no member groups inside a moments call) merges to it
     a = packed.forward(x.to(DEV), "ensemble", total_members=k, precision="bf16", member_begin=0,
                        member_count=10, output="moments")
@@ -960,7 +919,7 @@ def _large_bias_nets(width, n_hidden, k, d_in, bias_scale=20.0):
     nets = []
     for i in range(k):
         torch.manual_seed(7 + i)
-        net = build_network(_wide_arch(d_in, width, n_hidden, 1, bn=False)).eval()
+        net = build_network(wide_arch(d_in, width, n_hidden, 1, bn=False)).eval()
         with torch.no_grad():
             for m in net:
                 if isinstance(m, torch.nn.Linear):   # a dropped bias piece is an O(1) error
@@ -982,7 +941,7 @@ def test_bias_in_mma_matches_epilogue_bias_ensemble(width, n_hidden, k, n):
     out = _both_bias_variants(lambda: packed.forward(x.to(DEV), "ensemble", total_members=k,
                                                      precision="bf16"))
     for flag, (mean, std) in out.items():
-        _bf16_check(mean, std, ref_mean, ref_std, f"bias variant {flag}, {width}x{n_hidden}")
+        bf16_check(mean, std, ref_mean, ref_std, f"bias variant {flag}, {width}x{n_hidden}")
     # the two variants differ by accumulation order only
     scale = float(torch.as_tensor(ref_mean).abs().max() + torch.as_tensor(ref_std).abs().max())
     assert float((out["1"][0] - out["0"][0]).abs().max()) <= 2e-3 * scale
@@ -1002,7 +961,7 @@ def test_bias_in_mma_per_anchor_layer0_stages(width, n_hidden, k, n):
     # the last hidden activations alone is ~10 % of that spread (either variant), so the std is held
     # to the output scale (1e-2, measured 3e-4) and to half of its own scale only
     for flag, (mean, std) in out.items():
-        _bf16_check(mean, std, ref_mean, ref_std, f"bias variant {flag}, delta-uq {width}x{n_hidden}",
+        bf16_check(mean, std, ref_mean, ref_std, f"bias variant {flag}, delta-uq {width}x{n_hidden}",
                     tol_std=0.5)
     scale = float(torch.as_tensor(ref_mean).abs().max() + torch.as_tensor(ref_std).abs().max())
     assert float((out["1"][0] - out["0"][0]).abs().max()) <= 2e-3 * scale
@@ -1013,7 +972,7 @@ def test_bias_in_mma_per_anchor_layer0_stages(width, n_hidden, k, n):
                               anchors=anchors.to(DEV), member_begin=2, member_count=k - 2,
                               output="moments")
     ref_a = uq_oracle.delta_uq_forward(net, x, anchors[2:], k - 2)
-    _bf16_check(m_a, torch.sqrt(q_a / (k - 3)), ref_a[0], ref_a[1], "anchor shard", tol_std=0.5)
+    bf16_check(m_a, torch.sqrt(q_a / (k - 3)), ref_a[0], ref_a[1], "anchor shard", tol_std=0.5)
 
 
 @pytest.mark.parametrize("width,n_hidden,passes,n,final_drop", [
@@ -1043,4 +1002,4 @@ def test_bias_in_mma_with_live_dropout_philox_replay(width, n_hidden, passes, n,
     out = _both_bias_variants(lambda: packed.forward(x.to(DEV), "mc_dropout", total_members=passes,
                                                      precision="bf16", dropout_p=pdrop, seed=seed))
     for flag, (mean, std) in out.items():
-        _bf16_check(mean, std, ref_mean, ref_std, f"bias variant {flag}, mc-dropout {width}x{n_hidden}")
+        bf16_check(mean, std, ref_mean, ref_std, f"bias variant {flag}, mc-dropout {width}x{n_hidden}")

@@ -88,6 +88,51 @@ def injected_to_masks(flat, n, widths, total):
     return out
 
 
+def wide_arch(d_in, width, n_hidden, d_out, bn=True):
+    """``n_hidden`` x (Linear -> [BatchNorm1d] -> ReLU) of equal width, then Linear(width, d_out)."""
+    arch, prev = [], d_in
+    for _ in range(n_hidden):
+        arch.append({"Linear": {"args": [prev, width]}})
+        if bn:
+            arch.append({"BatchNorm1d": {"args": [width]}})
+        arch.append({"ReLU": {"inplace": True}})
+        prev = width
+    arch.append({"Linear": {"args": [prev, d_out]}})
+    return arch
+
+
+def randomise_bn(net, seed):
+    """Non-trivial eval-mode BatchNorm statistics, so that folding them into the weights matters."""
+    gen = torch.Generator().manual_seed(seed)
+    for m in net.modules():
+        if isinstance(m, torch.nn.BatchNorm1d):
+            m.running_mean.copy_(torch.randn(m.num_features, generator=gen) * 0.1)
+            m.running_var.copy_(torch.rand(m.num_features, generator=gen) + 0.5)
+
+
+def bf16_check(mean, std, ref_mean, ref_std, what, tol=1e-2, tol_std=5e-2):
+    """bf16 tolerance.  The natural unit is the magnitude of one member's output, taken as
+    ``scale = max|ref_mean| + max|ref_std|``: both errors must stay within ``tol * scale`` (measured
+    worst case over every bf16 test: 2.3e-3, and 4.3e-3 for identical passes whose std is 0 -- the
+    bound is 2.5-5x that; a mis-addressed K chunk is an error of >= 1/8 of scale), and the std
+    additionally within ``tol_std`` of its OWN scale (measured 1e-3 .. 2.2e-2; the largest values
+    belong to anchored nets whose spread is 16x smaller than their mean)."""
+    mean, std = mean.double().cpu(), std.double().cpu()
+    ref_mean, ref_std = torch.as_tensor(ref_mean).double(), torch.as_tensor(ref_std).double()
+    ms, ss = float(ref_mean.abs().max()), float(ref_std.abs().max())
+    scale = ms + ss
+    e_mean = float((mean - ref_mean).abs().max())
+    e_std = float((std - ref_std).abs().max())
+    print(f"[bf16 {what}] max|mean err| = {e_mean:.3e} ({e_mean / scale:.3e} of scale), "
+          f"max|std err| = {e_std:.3e} ({e_std / scale:.3e} of scale, "
+          f"{e_std / max(ss, 1e-30):.3e} of std scale)")
+    assert e_mean <= tol * scale, f"{what}: bf16 mean error {e_mean / scale:.3e} of scale > {tol}"
+    assert e_std <= tol * scale, f"{what}: bf16 std error {e_std / scale:.3e} of scale > {tol}"
+    if ss > 1e-3 * ms:   # identical passes have std == 0: nothing relative to check
+        assert e_std <= tol_std * ss, \
+            f"{what}: bf16 std error {e_std / ss:.3e} of std scale > {tol_std}"
+
+
 def assert_close_ref(got, ref, rtol, scale_ref=None, what=""):
     """|got - ref| <= rtol * |ref| + rtol * max|scale_ref|  (north_star's 1e-5 'relative', with the
     absolute floor tied to the output scale: std -> 0 in-distribution, SURVEY 8d)."""
