@@ -218,7 +218,23 @@ class MCDropoutModel(WrappedModelBase):
         self._injected_masks = None
 
     def _dropout_live(self) -> bool:
-        return any(isinstance(m, nn.Dropout) and m.training for m in self.model.modules())
+        """Whether the Dropouts are live.  The fused op applies ONE ``p`` (``dropout_percent``) and
+        ONE live flag to every Dropout, where the reference's ``self.model(x)`` honours each
+        module's own ``p`` and train / eval state: a Dropout that differs from the others is a
+        ``ValueError`` naming it, not a silently different result."""
+        drops = [(name, m) for name, m in self.model.named_modules() if isinstance(m, nn.Dropout)]
+        live = any(m.training for _, m in drops)
+        for name, m in drops:
+            if m.training != live:
+                raise ValueError(
+                    f"MCDropoutModel: Dropout {name!r} is in {'train' if m.training else 'eval'} "
+                    f"mode and another Dropout is not; the fused forward needs every Dropout live "
+                    "(after eval()) or every one in eval mode")
+            if live and m.p != self.dropout_percent:
+                raise ValueError(
+                    f"MCDropoutModel: Dropout {name!r} has p = {m.p}, not dropout_percent = "
+                    f"{self.dropout_percent}; the fused forward applies one p to every Dropout")
+        return live
 
     def inject_masks(self, masks: Optional[torch.Tensor]) -> None:
         """Testing hook: use these keep-masks (uint8, layout of ``uq_forward_args.masks``) instead
@@ -228,13 +244,14 @@ class MCDropoutModel(WrappedModelBase):
     def forward(self, x, return_ue=False):
         if self.training:
             return self.model(x)
+        live = self._dropout_live()
         ops._require_cuda(x, "x")
         packed = self._packed([self.model], x.device)
         # Philox stream keyed from torch's CPU generator: reproducible under torch.manual_seed
         seed = self._shared_seed(int(torch.randint(0, 2 ** 62, (1,)).item()), x.device)
         mean, std = self._fused(packed, x, "mc_dropout", int(self.num_samples),
                                 dropout_p=float(self.dropout_percent),
-                                dropout_active=self._dropout_live(), seed=seed,
+                                dropout_active=live, seed=seed,
                                 masks=self._injected_masks)
         return (mean, std) if return_ue else mean
 

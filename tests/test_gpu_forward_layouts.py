@@ -4,9 +4,8 @@
 Each case builds its networks, computes ONE float64 reference (``copy.deepcopy(net).double()``,
 float64 inputs / anchors / targets, the dtype-generic ``oracle.uq_oracle``; native Philox masks are
 exported and replayed) and checks every precision against it in the same body.  Every forward also
-runs under ``torch.profiler``: the kernel instantiation it launched must be the one
-``expected_kernels`` restates from the dispatch in ``csrc/mlp_tc.cu`` (``tc_forward``),
-``mlp_tc2.cu`` (``tc2_launch``) and ``mlp_tcx.cu`` (``tcx_plan``), so that no case silently stops
+runs under ``torch.profiler``: the kernel instantiations it launched must be the ones
+``tests.util.expected_kernels`` restates from the dispatch code, so that no case silently stops
 covering its kernel when the dispatch changes.
 
 Layer 0 of the bf16 kernels packs ``[x_hi | x_lo | x_hi] . [w_hi | w_hi | w_lo]`` into one K <= 64
@@ -20,7 +19,6 @@ mean's scale), ``bf16_check`` for bf16, and for the bf16-exact one-layer nets of
 ``test_layer0_input_bits_bf16`` a bound per ``s`` set at ~4x the measured worst case.
 """
 import copy
-import re
 
 import pytest
 import torch
@@ -29,12 +27,12 @@ from nnueehcs_b200 import ops
 from nnueehcs_b200.model_builder import (DeltaUQMLPModelBuilder, EnsembleModelBuilder,
                                          build_network)
 from oracle import uq_oracle
-from tests.util import (assert_close_ref, bf16_check, delta_arch, injected_to_masks,
-                        mc_arch_with_dropout, randomise_bn, wide_arch)
+from tests.util import (RTOL32, assert_close_ref, assert_live_spread, bf16_check, check,
+                        delta_arch, injected_to_masks, mc_arch_with_dropout, pager_reference,
+                        randomise_bn, run, wide_arch)
 
 pytestmark = pytest.mark.gpu
 DEV = torch.device("cuda:0")
-RTOL32 = 1e-5
 N = 259                   # two 128-row tiles + 3 rows; four 64-row tiles + 3 rows
 WIDTHS = [128, 320, 1024]
 P_DROP, PASSES, ENSEMBLE_K, ANCHORS = 0.2, 5, 3, 5
@@ -49,48 +47,6 @@ def split_factor(d_in):
     return s
 
 
-def expected_kernels(precision, mode, width, d_in, d_out, live_dropout):
-    """The forward kernel instantiations one call launches, as ``family<args>`` strings.
-
-    ``d_in`` is the NETWORK input width (twice the sample width for Delta-UQ / PAGER).  Restates
-    ``tc_forward`` (mlp_tc.cu), ``tc2_launch`` / ``dispatch_h3`` / ``tc4_launch`` (the bias-in-the-MMA
-    variants are the default for d_out 1), ``tcx_plan`` (mlp_tcx.cu: hidden width <= 512 and at most
-    16 network inputs) and ``fp32_forward`` (mlp_fp32.cu: the vectorised loader needs a multiple of
-    4 inputs)."""
-    b = lambda v: "true" if v else "false"
-    dpad = 1 if d_out == 1 else 8
-    mc = live_dropout and mode == "mc_dropout"
-    if precision == "bf16":
-        if width > 512:
-            return {f"tc3<{width},1,true>" if dpad == 1 else f"tc3<{width},8,false>"}
-        if width in (64, 128) and dpad == 1:
-            return {f"tc4<{width},true,{b(mc)}>"}
-        return {f"tc2<{width},{dpad},2,{b(mc)},{b(dpad == 1)}>"}
-    if precision == "fp32" and width <= 512 and d_in <= 16:
-        if width in (64, 128) and dpad == 1:
-            return {f"tcx4<{width},{b(mc)}>"}
-        return {f"tcx<{width},{dpad},{b(mc)}>"}
-    return {f"sgemm_tn_kernel<{b(d_in % 4 == 0)}>", "sgemm_tn_kernel<true>"}
-
-
-_KERNEL = re.compile(r"\b(?:uq_mlp_(tc2|tc3|tc4|tcx|tcx4)_kernel|(sgemm_tn_kernel))\s*<([^<>]*)>")
-
-
-def forward_kernels(call):
-    """Run ``call()`` under the CUDA profiler; return its result and the forward kernels it ran."""
-    with torch.profiler.profile(activities=[torch.profiler.ProfilerActivity.CUDA]) as prof:
-        out = call()
-        torch.cuda.synchronize()
-    names = [e.name for e in prof.events() if e.device_type == torch.autograd.DeviceType.CUDA]
-    assert names, "the profiler recorded no CUDA kernel at all: kernel attribution is impossible"
-    found = set()
-    for name in names:
-        m = _KERNEL.search(name)
-        if m:
-            found.add(f"{m.group(1) or m.group(2)}<{re.sub(r'\s+', '', m.group(3))}>")
-    return out, found
-
-
 @pytest.fixture(scope="module")
 def seen():
     """Every forward kernel instantiation this file ran, printed at the end."""
@@ -99,38 +55,10 @@ def seen():
     print("\n[forward layouts] kernel instantiations run:\n  " + "\n  ".join(sorted(names)))
 
 
-def run(seen, packed, precision, what, x, mode, live_dropout=False, **kw):
-    """``packed.forward`` with kernel attribution."""
-    (a, b), found = forward_kernels(lambda: packed.forward(x, mode, precision=precision, **kw))
-    width = packed.signature[0][1]
-    expect = expected_kernels(precision, mode, width, packed.d_in, packed.d_out, live_dropout)
-    assert found == expect, f"{what} [{precision}]: ran {sorted(found)}, dispatch says {sorted(expect)}"
-    seen.update(found)
-    return a, b
-
-
-def check(precision, mean, std, ref_mean, ref_std, what):
-    if precision == "bf16":
-        bf16_check(mean, std, ref_mean, ref_std, what)
-        return
-    e_mean = float((mean.double().cpu() - ref_mean).abs().max())
-    e_std = float((std.double().cpu() - ref_std).abs().max())
-    print(f"[{precision} {what}] max|mean err| = {e_mean:.3e}, max|std err| = {e_std:.3e} "
-          f"(mean scale {float(ref_mean.abs().max()):.3e})")
-    assert_close_ref(mean, ref_mean, RTOL32, what=f"{what} mean")
-    assert_close_ref(std, ref_std, RTOL32, scale_ref=ref_mean, what=f"{what} std")
-
-
 def check_moments(precision, mean, m2, count, ref_mean, ref_std, what):
     """``output='moments'`` of ``count`` members against the float64 (mean, std) of that range."""
     check(precision, mean, torch.sqrt(m2.double().clamp_min(0) / (count - 1)), ref_mean, ref_std,
           what + " moments")
-
-
-def assert_live_spread(ref_mean, ref_std, what):
-    """A std check means nothing when the members agree: the reference must spread."""
-    ms, ss = float(ref_mean.abs().max()), float(ref_std.abs().max())
-    assert ss >= 1e-2 * ms, f"{what}: reference std {ss:.3e} < 1e-2 of mean scale {ms:.3e}"
 
 
 def make_nets(arch, k, seed, bn=True):
@@ -175,16 +103,6 @@ def mc_case(d_in, width, d_out, seed):
     ref_tail = uq_oracle.mc_dropout_forward(net64, x64, PASSES - 1, P_DROP, masks=masks[1:])
     ref_off = uq_oracle.mc_dropout_forward(net64, x64, PASSES, P_DROP, dropout_active=False)
     return packed, x, ref, ref_tail, ref_off
-
-
-def pager_reference(net64, x64, a64, ys64, anchor_first):
-    """(mean over anchors of the swapped-role predictions, max_k |P[k] - Y_k|) for any d_out."""
-    with torch.no_grad():
-        p = torch.stack([uq_oracle.sequential_forward(
-            net64, uq_oracle.anchored_input(a64[j:j + 1].expand(x64.shape[0], -1), x64,
-                                            anchor_first))
-            for j in range(a64.shape[0])])                                # [K, N, d_out]
-    return p.mean(0), (p - ys64.unsqueeze(1)).abs().max(dim=0)[0]
 
 
 def anchored_case(dx, width, d_out, seed, anchor_first):
